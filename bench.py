@@ -24,6 +24,10 @@ kernel, roofline and — on rank 0 at N=1 — cpu_baseline:
   "5"  avg_over_time wide-events scan: 12.5 M rows x 32 f64 columns per GPU (100 M rows over 8 GPUs): K6 per-column
        (sum, count) + for N>1 the all-reduce of the 32 x 2 scalars.
 Inputs are far larger than L2 (126 MB) in every config, so no explicit L2 flush is needed between steps.
+
+--dump-outputs DIR writes, after the timed steps, what each timed path returned in its last timed step as DIR/<name>.npy
+(a fixed, seeded sample of the rows of the larger results; see OutputDump).  Every input is generated from SEED, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +43,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 T0 = 1_700_000_000_000
 N_SAMPLES = 1000
@@ -66,6 +71,69 @@ def load_traffic(key="range_lean_kernel"):
         return float(d[key]["dram_bytes_per_sample"]), f"profiles/r2_traffic.json[{key}] ({d[key].get('kernel', '')})"
     except Exception:
         return None, None
+
+
+class OutputDump:
+    """--dump-outputs DIR: the results of the last timed step of each timed path, as DIR/<name>.npy.
+
+    A [rows x T] result is sampled: a fixed, seeded choice of rows (the same for every run with the same arguments),
+    written as <name>_rows (row indices), <name>_out (f64 values, 0.0 where there is no value) and <name>_valid (f32
+    0/1 per slot, unpacked from the validity bit words).  Counts are written as f64.  All files together stay below
+    LIMIT bytes.  Only rank 0 writes (its own shard)."""
+    LIMIT = 64_000_000
+
+    def __init__(self, path, rank=0):
+        self.path = path if rank == 0 else None
+        self.bytes = 0
+        if self.path:
+            os.makedirs(self.path, exist_ok=True)
+
+    @staticmethod
+    def sample(n, k):
+        import numpy as np
+        if n <= k:
+            return np.arange(n, dtype=np.int64)
+        return np.sort(np.random.default_rng(SEED).choice(n, k, replace=False)).astype(np.int64)
+
+    @staticmethod
+    def _rows(a, idx, shape):
+        """rows idx of `a` viewed as `shape` -> numpy; `a` is a numpy array or a torch tensor (device or host)."""
+        if hasattr(a, "index_select"):
+            import torch
+            return a.reshape(shape).index_select(0, torch.from_numpy(idx).to(a.device)).cpu().numpy()
+        return a.reshape(shape)[idx]
+
+    def put(self, name, a):
+        import numpy as np
+        if not self.path:
+            return
+        a = np.ascontiguousarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        self.bytes += a.nbytes
+        if self.bytes > self.LIMIT:
+            raise RuntimeError(f"--dump-outputs: {name} takes the dump past {self.LIMIT} bytes")
+        np.save(os.path.join(self.path, name + ".npy"), a)
+
+    def result(self, name, out, valid, n_rows, T, k):
+        """A sample of k rows of an [n_rows x T] f64 result and its [n_rows x ceil(T / 32)] u32 validity words."""
+        import numpy as np
+        if not self.path:
+            return
+        idx = self.sample(n_rows, k)
+        words = self._rows(valid, idx, (n_rows, (T + 31) // 32)).view(np.uint32)
+        self.put(name + "_rows", idx.astype(np.float64))
+        self.put(name + "_out", self._rows(out, idx, (n_rows, T)).astype(np.float64))
+        self.put(name + "_valid", np.unpackbits(words.view(np.uint8), axis=1, bitorder="little")[:, :T].astype(np.float32))
+
+    def groups(self, name, vals, cnt, n_rows, T, k):
+        """A sample of k rows of an [n_rows x T] (f64 value, u32 count) pair."""
+        import numpy as np
+        if not self.path:
+            return
+        idx = self.sample(n_rows, k)
+        self.put(name + "_rows", idx.astype(np.float64))
+        self.put(name + "_out", self._rows(vals, idx, (n_rows, T)).astype(np.float64))
+        self.put(name + "_count", self._rows(cnt, idx, (n_rows, T)).view(np.uint32).astype(np.float64))
 
 
 class ClockSampler:
@@ -215,9 +283,11 @@ def run_reference(args):
     t = 0.0
     samples = 0
     for _ in range(args.steps):
-        dt, n, _, _ = cpu_reference_pass(per_step, cores)
+        dt, n, out, valid = cpu_reference_pass(per_step, cores)
         t += dt
         samples += n
+    if args.dump_outputs:
+        OutputDump(args.dump_outputs).result("rate", out, valid, per_step, N_SAMPLES, 2048)
     value = samples / t
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -302,6 +372,7 @@ class Harness:
                              "use --impl reference for the CPU arm")
         torch.cuda.set_device(self.local)
         self.dev = torch.device("cuda", self.local)
+        self.dump = OutputDump(args.dump_outputs, self.rank) if args.dump_outputs else None
         if self.world > 1:
             dist.init_process_group("nccl", device_id=self.dev)
         self.ctx = Context(self.local)
@@ -388,6 +459,8 @@ def bench_config2(h: Harness, sampler):
         ctx.synth_fill_dev(h.rank * S, S, N_SAMPLES, T0, SCRAPE, args.jitter_variant_ms, args.resets, SEED, ts, val, sid)
         ctx.sync()
         jms, _, _ = h.timed(step, args.steps, args.warmup)
+        if h.dump:
+            h.dump.result("rate_jitter", out, valid, S, T, 512)
         jitter_variant = {"jitter_ms": args.jitter_variant_ms, "ms_per_step": jms,
                           "value": n_rows * h.world / (jms * 1e-3), "unit": UNIT,
                           "warp_tier_series": ctx.last_warp_tier_series(), "slow_path_series": ctx.last_slow_series()}
@@ -395,6 +468,8 @@ def bench_config2(h: Harness, sampler):
     ctx.sync()
 
     ms, launches, window = h.timed(step, args.steps, args.warmup)
+    if h.dump:
+        h.dump.result("rate", out, valid, S, T, 2048)
     slow_series, warp_tier_series = ctx.last_slow_series(), ctx.last_warp_tier_series()
     clocks = sampler.stop(*window) if sampler else None
     st = h.stage_ms(step, (0, 1), reps=min(args.steps, 5))
@@ -449,6 +524,8 @@ def bench_config2(h: Harness, sampler):
         torch.cuda.synchronize()
         dt_off = h.max_over_ranks(time.perf_counter() - t0)
         h2d_off = ctx.last_h2d_bytes()
+        if h.dump:
+            h.dump.result("rate_e2e", h_out, h_valid, Se, T, 512)
         res["e2e"] = {"value": Se * N_SAMPLES * h.world * n_e2e / dt, "unit": UNIT,
                       "h2d_bytes_per_step": h2d_ids, "d2h_bytes_per_step": Se * T * 8 + Se * Tw * 4,
                       "host_columns_bytes_per_step": Se * N_SAMPLES * 20,
@@ -494,8 +571,10 @@ def bench_config3(h: Harness):
         ctx.series_offsets_dev(sid, n_rows, S, offsets)
         ctx.range_group_sum_allreduce_dev(p, ts, val, offsets, n_rows, S, ix, tiles, gsum, gcnt)
 
-    steps = max(3, args.steps // 2) if args.steps > 4 else args.steps
+    steps = args.steps
     ms, launches, _ = h.timed(step, steps, max(3, args.warmup))
+    if h.dump:
+        h.dump.groups("sumby", gsum, gcnt, G, T, 512)
     st = h.stage_ms(step, (0, 1, 4))
     # compute-only variant of the same step (no collective) on N>1, to name the collective's share
     ms_nocoll = None
@@ -564,8 +643,10 @@ def bench_config4(h: Harness):
         ctx.range_eval_dev(p, ts, val, offsets, n_rows, S, rates, rvalid)
         ctx.histogram_quantile_dev(0.99, le, B, rates, rvalid, H, T, out, ovalid)
 
-    steps = max(3, h.args.steps // 2) if h.args.steps > 4 else h.args.steps
+    steps = args.steps
     ms, launches, _ = h.timed(step, steps, max(3, args.warmup))
+    if h.dump:
+        h.dump.result("hist", out, ovalid, H, T, 4096)
     st = h.stage_ms(step, (0, 1, 3))
     peak, _ = load_peaks()
     alg_range = 16.0 * n_rows + 8.0 * S * T + 4.0 * S * Tw + 8.0 * (S + 1)
@@ -595,7 +676,9 @@ def bench_config5(h: Harness):
     """avg_over_time wide-events scan: per-column (sum, count) of 32 f64 columns + (N>1) the all-reduce of the scalars."""
     torch, args, ctx, dev = h.torch, h.args, h.ctx, h.dev
     rows, cols = args.wide_rows_per_gpu, 32
-    data = torch.rand((cols, rows), dtype=torch.float64, device=dev)
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(SEED + h.rank)   # the same table on every run
+    data = torch.rand((cols, rows), dtype=torch.float64, device=dev, generator=gen)
     data[:, ::1009] = float("nan")     # stale markers are skipped like SeriesNormalize's filter
     ptrs = torch.tensor([data[c].data_ptr() for c in range(cols)], dtype=torch.int64, device=dev)
     col_sum = torch.zeros(cols, dtype=torch.float64, device=dev)
@@ -607,8 +690,11 @@ def bench_config5(h: Harness):
         ctx.column_reduce_dev(ptrs, cols, rows, col_sum, col_cnt)
         ctx.allreduce_columns_dev(col_sum, col_cnt, cols)
 
-    steps = max(3, h.args.steps // 2) if h.args.steps > 4 else h.args.steps
+    steps = args.steps
     ms, launches, _ = h.timed(step, steps, max(3, args.warmup))
+    if h.dump:
+        h.dump.put("wide_sum", col_sum.cpu().numpy())
+        h.dump.put("wide_count", col_cnt.cpu().numpy().astype("float64"))
     st = h.stage_ms(step, (3, 4))
     avg = (col_sum / col_cnt.to(torch.float64)).cpu()
     peak, _ = load_peaks()
@@ -749,6 +835,9 @@ def main():
                     help="config 3, N>1: group ranges the partials are computed and all-reduced in (overlap)")
     ap.add_argument("--hist-per-gpu", type=int, default=125_000)
     ap.add_argument("--wide-rows-per-gpu", type=int, default=12_500_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what each timed path returned in its last step as DIR/<name>.npy "
+                         f"(f32 / f64, a seeded sample of rows, at most {OutputDump.LIMIT} bytes in all)")
     args = ap.parse_args()
     global JITTER_MS
     JITTER_MS = args.jitter_ms

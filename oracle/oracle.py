@@ -44,9 +44,14 @@ def _cpu_stamp() -> str:
         return "unknown"
 
 
+_SOURCES = ("promql_oracle.c", "promql_oracle.h", "Makefile")
+
+
 def build(force: bool = False) -> str:
-    """Compile the oracle with gcc (oracle/Makefile).  Building the checker is not using it."""
-    src = [os.path.join(_HERE, f) for f in ("promql_oracle.c", "promql_oracle.h", "Makefile")]
+    """Compile the oracle with gcc (oracle/Makefile).  Building the checker is not using it.  -> path of the library.
+    In a source tree that cannot be written (a read-only checkout) a library that has to be rebuilt is compiled into a
+    temporary directory instead, removed again when the process exits."""
+    src = [os.path.join(_HERE, f) for f in _SOURCES]
     stamp_path = _SO + ".cpu"
     stamp = _cpu_stamp()
     try:
@@ -54,10 +59,24 @@ def build(force: bool = False) -> str:
     except OSError:
         same_cpu = False
     if force or not same_cpu or not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in src):
+        if not os.access(_HERE, os.W_OK):
+            return _build_private()
         subprocess.check_call(["make", "-s", "-B", "-C", _HERE, "liboracle.so"])
         with open(stamp_path, "w") as f:
             f.write(stamp)
     return _SO
+
+
+def _build_private() -> str:
+    import atexit
+    import shutil
+    import tempfile
+    tmp = tempfile.mkdtemp(prefix="promql_oracle_")
+    atexit.register(shutil.rmtree, tmp, True)
+    for f in _SOURCES:
+        shutil.copy(os.path.join(_HERE, f), tmp)
+    subprocess.check_call(["make", "-s", "-B", "-C", tmp, "liboracle.so"])
+    return os.path.join(tmp, "liboracle.so")
 
 
 class Params(C.Structure):
@@ -72,8 +91,7 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_SO)
+        L = C.CDLL(build())
         i64p, f64p, u32p, u64p, u8p = (C.POINTER(C.c_int64), C.POINTER(C.c_double), C.POINTER(C.c_uint32),
                                        C.POINTER(C.c_uint64), C.POINTER(C.c_uint8))
         L.orc_num_steps.restype = C.c_int64
