@@ -143,13 +143,22 @@ __global__ void __launch_bounds__(256) group_finalize_kernel(int32_t agg, double
   }
 }
 
-// Cross-rank merge helpers of the by-label partials (b2p_allreduce_partials_dev).
-// phase 0: groups this rank has no row for become the neutral element of min / max; phase 1 (after the all-reduce,
-// cnt = global count): groups absent everywhere read 0.0 again, like a freshly built partial.
-__global__ void __launch_bounds__(256) minmax_neutral_kernel(bool is_min, double* val, const uint32_t* cnt, uint64_t n, int phase) {
-  const double inf = __longlong_as_double(0x7ff0000000000000ll);
+// Cross-rank merge helpers of the by-label partials (b2p_allreduce_partials_dev).  min / max are reduced as total-order
+// keys (int64 min / max on the collective), so NaNs of either sign and signed zeros merge exactly like the by-label
+// kernel's own fold; an f64 min / max there would depend on the rank order.
+// encode: val[i] becomes total_key(val[i]) in place, or the neutral key (INT64_MAX for min, INT64_MIN for max) for a
+// group this rank has no row for.  decode (after the all-reduce, cnt = global count): keys turn back into values
+// (total_key is its own inverse) and groups absent everywhere read 0.0 again, like a freshly built partial.
+__global__ void __launch_bounds__(256) minmax_key_encode_kernel(bool is_min, double* val, const uint32_t* cnt, uint64_t n) {
+  long long* key = reinterpret_cast<long long*>(val);
+  const long long neutral = is_min ? 0x7fffffffffffffffll : (long long)0x8000000000000000ull;
   for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
-    if (cnt[i] == 0) val[i] = phase == 0 ? (is_min ? inf : -inf) : 0.0;
+    key[i] = cnt[i] ? total_key(val[i]) : neutral;
+}
+__global__ void __launch_bounds__(256) minmax_key_decode_kernel(double* val, const uint32_t* cnt, uint64_t n) {
+  const long long* key = reinterpret_cast<const long long*>(val);
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+    val[i] = cnt[i] ? __longlong_as_double(total_key(__longlong_as_double(key[i]))) : 0.0;
 }
 // (cnt, mean, M2) states of population variance.  phase 0: wsum = cnt * mean, cnt_r = cnt (kept: cnt becomes global);
 // phase 1 (wsum, cnt all-reduced): mean_g = wsum / cnt; M2 += cnt_r * (mean_r - mean_g)^2 — the all-reduce of M2 that

@@ -53,7 +53,7 @@ struct Nccl {
   typedef struct ncclComm* comm_t;
   struct unique_id { char internal[128]; };
   enum { kSum = 0, kMax = 2, kMin = 3 };
-  enum { kUint32 = 3, kUint64 = 5, kFloat64 = 8 };
+  enum { kUint32 = 3, kInt64 = 4, kUint64 = 5, kFloat64 = 8 };
   int (*GetUniqueId)(unique_id*) = nullptr;
   int (*CommInitRank)(comm_t*, int, unique_id, int) = nullptr;
   int (*CommDestroy)(comm_t) = nullptr;
@@ -1307,8 +1307,8 @@ int b2p_comm_destroy(b2p_ctx* c) {
 // One all-reduce of the by-label partials [n] of every rank, enqueued on the context's stream (asynchronous).
 //   SUM / AVG / COUNT   val (plain sums) and cnt are added (the __sum_state / __sum_merge split of the reference,
 //                       src/query/src/dist_plan/commutativity.rs:85-113); finalise afterwards (b2p_group_finalize_dev)
-//   MIN / MAX           cnt is added, val is reduced with min / max after groups absent on a rank (cnt == 0) were
-//                       set to +inf / -inf; groups absent everywhere end up 0.0 again
+//   MIN / MAX           cnt is added, val is reduced as f64::total_cmp keys with int64 min / max (groups absent on a
+//                       rank, cnt == 0, hold the neutral key); groups absent everywhere end up 0.0 again
 //   STDDEV / STDVAR     inputs are per-rank (cnt, mean, M2 = val): the global mean comes from an all-reduce of
 //                       cnt*mean, then M2 = sum_r [M2_r + cnt_r (mean_r - mean)^2] (commutativity.rs:158-191 merges
 //                       the same state pairwise); on return mean / val hold the merged state on every rank
@@ -1327,12 +1327,12 @@ int b2p_allreduce_partials_dev(b2p_ctx* c, int32_t agg, double* val, uint32_t* c
   uint64_t blocks = (n + 255) / 256;
   if (blocks > (uint64_t)c->num_sms * 16) blocks = (uint64_t)c->num_sms * 16;
   if (agg == B2P_AGG_MIN || agg == B2P_AGG_MAX) {
-    minmax_neutral_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(agg == B2P_AGG_MIN, val, cnt, n, 0);
+    minmax_key_encode_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(agg == B2P_AGG_MIN, val, cnt, n);
     NCCL_TRY(g_nccl.GroupStart());
-    NCCL_TRY(g_nccl.AllReduce(val, val, n, Nccl::kFloat64, agg == B2P_AGG_MIN ? Nccl::kMin : Nccl::kMax, c->comm, c->stream));
+    NCCL_TRY(g_nccl.AllReduce(val, val, n, Nccl::kInt64, agg == B2P_AGG_MIN ? Nccl::kMin : Nccl::kMax, c->comm, c->stream));
     NCCL_TRY(g_nccl.AllReduce(cnt, cnt, n, Nccl::kUint32, Nccl::kSum, c->comm, c->stream));
     NCCL_TRY(g_nccl.GroupEnd());
-    minmax_neutral_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(agg == B2P_AGG_MIN, val, cnt, n, 1);
+    minmax_key_decode_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(val, cnt, n);
     c->launches += 2;
   } else if (var) {
     int rc;

@@ -67,22 +67,31 @@ def finalize_host(agg: str, sum_a: np.ndarray, cnt_a: np.ndarray) -> np.ndarray:
     return out
 
 
+def total_key(bits):
+    """f64::total_cmp key of float64 values viewed as int64 (torch tensor): an int64 whose signed order is the total
+    order of the floats (-NaN < -inf < ... < -0.0 < +0.0 < ... < +inf < +NaN).  The map is its own inverse."""
+    return bits ^ ((bits >> 63) & 0x7FFFFFFFFFFFFFFF)
+
+
 def merge_partials(agg: str, val_t, cnt_t, mean_t=None, group=None):
     """Host mirror of b2p_allreduce_partials_dev (same formulas, torch.distributed instead of the library's NCCL
     communicator; used by the gloo tests): in-place merge of every rank's by-label partials.
       sum / avg / count : val and cnt are added                       (commutativity.rs:85-113)
-      min / max         : groups absent on a rank (cnt == 0) are neutral (+inf / -inf), val is reduced with
-                          min / max, cnt is added, groups absent everywhere read 0.0 again
+      min / max         : val is reduced as total-order keys (int64 min / max), so NaNs of either sign and signed
+                          zeros merge like the single-rank by-label min / max (f64 min / max would depend on the
+                          rank order there); groups absent on a rank (cnt == 0) hold the neutral key (INT64_MAX /
+                          INT64_MIN), cnt is added, groups absent everywhere read 0.0 again
       stddev / stdvar   : per-rank (cnt, mean, M2 = val) states; global mean from an all-reduce of cnt * mean,
                           M2 = sum_r [M2_r + cnt_r (mean_r - mean)^2]  (commutativity.rs:158-191)"""
     import torch
     import torch.distributed as dist
     cnt64 = cnt_t.to(torch.int64)
     if agg in ("min", "max"):
-        neutral = float("inf") if agg == "min" else float("-inf")
-        val_t[cnt64 == 0] = neutral
-        dist.all_reduce(val_t, op=dist.ReduceOp.MIN if agg == "min" else dist.ReduceOp.MAX, group=group)
+        key = total_key(val_t.contiguous().view(torch.int64))
+        key[cnt64 == 0] = torch.iinfo(torch.int64).max if agg == "min" else torch.iinfo(torch.int64).min
+        dist.all_reduce(key, op=dist.ReduceOp.MIN if agg == "min" else dist.ReduceOp.MAX, group=group)
         dist.all_reduce(cnt64, op=dist.ReduceOp.SUM, group=group)
+        val_t.copy_(total_key(key).view(torch.float64))
         val_t[cnt64 == 0] = 0.0
     elif agg in ("stddev", "stdvar"):
         cnt_r = cnt64.clone()

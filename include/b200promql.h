@@ -212,7 +212,7 @@ B2P_API int b2p_comm_unique_id(void* out_id, size_t bytes);
 B2P_API int b2p_comm_init(b2p_ctx* ctx, const void* id, size_t bytes, int n_ranks, int rank);
 B2P_API int b2p_comm_destroy(b2p_ctx* ctx);
 /* In-place merge of every rank's partials [n] on the context's stream (asynchronous): SUM / AVG / COUNT add val and
- * cnt; MIN / MAX reduce val with min / max (groups absent on a rank are neutral) and add cnt; STDDEV / STDVAR merge
+ * cnt; MIN / MAX reduce val in the f64::total_cmp order (int64 keys; groups absent on a rank are neutral) and add cnt; STDDEV / STDVAR merge
  * the (cnt, mean, M2 = val) states.  A context without communicator and n_ranks == 1 returns at once. */
 B2P_API int b2p_allreduce_partials_dev(b2p_ctx* ctx, int32_t agg, double* val, uint32_t* cnt, double* mean, uint64_t n);
 /* Wide avg_over_time (config 5): per-column (sum, count) of every rank added in place. */

@@ -3,7 +3,8 @@ tests/test_multi_gpu.py when at least two GPUs are visible):
 
   * sum by (..)(rate(..)) with series hash-sharded over the ranks, through b2p_range_group_sum_allreduce_dev (fused
     partials, tiles all-reduced on the library's NCCL communicator) == the oracle on the unsharded data;
-  * b2p_allreduce_partials_dev for min / max and for the (count, mean, M2) states of stddev / stdvar == the oracle.
+  * b2p_allreduce_partials_dev for min / max (bit for bit, with NaNs of both signs, signed zeros and infinities among
+    the members) and for the (count, mean, M2) states of stddev / stdvar == the oracle.
 torch.distributed only carries the 128-byte communicator id and the final verdict."""
 import os
 import sys
@@ -66,13 +67,29 @@ def main():
     ctx.range_eval_dev(p, d_ts, d_val, d_off, rows.size, ns, out, valid)
     ctx.sync()
     scale = float(np.abs(full_out).max())
+    # min / max also merge NaNs of both signs, signed zeros and infinities: a quarter of the cells of every series hold
+    # one of them, so most (group, step) cells see several on different ranks, where only the total order decides
+    spec = np.concatenate([np.array([0x0, 0x8000000000000000, 0x7FF0000000000000, 0xFFF0000000000000,
+                                     0x7FF8000000000000, 0xFFF8000000000000, 0x7FF0000000000002, 0x1],
+                                    np.uint64).view(np.float64), [1e308, -1e308]])
+
+    def specialize(a, series):
+        a = a.copy()
+        k = np.arange(T)[None, :] + series[:, None]
+        hit = (k + 2 * series[:, None]) % 4 == 0
+        a[hit] = spec[(k % spec.size)[hit]]
+        return a
+
+    full_mm = specialize(full_out, np.arange(S))
+    out_mm = torch.from_numpy(specialize(out.cpu().numpy().reshape(ns, T), owned).reshape(-1)).to(dev)
     for agg in ("min", "max", "stddev", "stdvar", "avg"):
-        e_val, e_c = orc.group_aggregate(agg, full_out, full_valid, gid, G)
+        mm = agg in ("min", "max")
+        e_val, e_c = orc.group_aggregate(agg, full_mm if mm else full_out, full_valid, gid, G)
         pv = torch.zeros(G * T, dtype=torch.float64, device=dev)
         pc = torch.zeros(G * T, dtype=torch.int32, device=dev)
         pm = torch.zeros(G * T, dtype=torch.float64, device=dev)
         var = agg in ("stddev", "stdvar")
-        ctx.group_aggregate_partial_dev(agg, out, valid, d_gid, ns, G, T, pv, pc, pm if var else None)
+        ctx.group_aggregate_partial_dev(agg, out_mm if mm else out, valid, d_gid, ns, G, T, pv, pc, pm if var else None)
         ctx.allreduce_partials_dev(agg, pv, pc, pm if var else None, G * T)
         if agg in ("stddev", "stdvar", "avg"):
             ctx.group_finalize_dev(agg, pv, pc, G * T)
@@ -80,8 +97,8 @@ def main():
         got, cnt = pv.cpu().numpy().reshape(G, T), pc.cpu().numpy().view(np.uint32).reshape(G, T)
         ok = ok and bool((cnt == e_c).all())
         m = e_c > 0
-        if agg in ("min", "max"):
-            ok = ok and bool((got[m] == e_val[m]).all())
+        if mm:
+            ok = ok and bool((got.view(np.uint64)[m] == e_val.view(np.uint64)[m]).all())
         else:
             err = np.abs(got[m] - e_val[m])
             bad = (err > 1e-9 * np.maximum(np.abs(e_val[m]), 1e-300)) & (err > 1e-9 * scale)
